@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]              # this repo (CUDA kernels)
   python bench.py --impl reference [--gpus N] [--steps K] ...      # the reference's CPU pipeline
+  python bench.py ... --dump-outputs DIR                           # + what the last timed step returned, as DIR/*.npy
 
 Metric (BASELINE.json): ELF-strip GB/s of build-tree `.so` INPUT bytes.
 
@@ -53,6 +54,13 @@ FILES_PER_GPU = 1250
 SEED = 0xB200
 SAMPLE_SPAN = 15 << 30        # host-side legs (e2e, tree, CPU baseline) work on the first <= 15 GiB of a shard
 LAUNCHES_PER_BATCH = 3        # plan, scan (+ tile expansion of the very big extents), compaction
+# --dump-outputs: the stripped bytes of a whole shard are tens of GB, so a fixed, seeded sample of them is written:
+# DUMP_FILES outputs, each by its two ends (ELF and program headers; section table and .shstrtab) and DUMP_WINDOWS
+# windows of its body.  At most 64 x 64 KiB bytes = 16 MiB as float32.
+DUMP_SEED = 0xD0B
+DUMP_FILES = 64
+DUMP_EDGE = 16 << 10
+DUMP_WINDOWS, DUMP_WINDOW = 8, 4 << 10
 
 
 def peaks():
@@ -296,6 +304,35 @@ def workload_config(a, world):
             "l2": "inputs (>10 GB per GPU) far larger than the 126 MB L2; no flush needed"}
 
 
+def dump_files(n):
+    """Indices of the outputs whose bytes --dump-outputs samples: the same for every run of a shard of n files."""
+    import numpy as np
+    return sorted(int(i) for i in np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_FILES), replace=False))
+
+
+def dump_sample(i, out):
+    """Both ends of output i and DUMP_WINDOWS seeded windows of its body, concatenated."""
+    import numpy as np
+    b = np.frombuffer(out, dtype=np.uint8)
+    parts = [b[:DUMP_EDGE], b[-DUMP_EDGE:]]
+    if len(b) > DUMP_WINDOW:
+        starts = np.random.default_rng([DUMP_SEED, i]).integers(0, len(b) - DUMP_WINDOW + 1, size=DUMP_WINDOWS)
+        parts += [b[s:s + DUMP_WINDOW] for s in starts]
+    return np.concatenate(parts)
+
+
+def write_dump(d, out_sizes, status, files, outputs):
+    """DIR/<name>.npy: per-file output sizes and status codes, the sampled file indices and their sampled bytes."""
+    import numpy as np
+    arrays = {"out_sizes": out_sizes.astype(np.float64), "status": status.astype(np.float64),
+              "sample_files": np.array(files, dtype=np.float64),
+              "sample_bytes": np.concatenate([dump_sample(i, outputs[i]) for i in files]).astype(np.float32)}
+    assert sum(x.nbytes for x in arrays.values()) <= 64 << 20
+    os.makedirs(d, exist_ok=True)
+    for name, x in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), x)
+
+
 def _materialize(args):
     corpus, i, path = args
     with open(path, "wb") as f:
@@ -522,20 +559,27 @@ def run_b200(a, rank, local_rank, world):
         return 0
 
     # ---- parity on the shard that was benchmarked: 8 size-stratified files per rank vs the real GNU strip
+    last_sizes, last_status = batch.out_sizes[:n].copy(), batch.status[:n].copy()   # as the last timed step returned them
     order = np.argsort(batch.sizes[:n], kind="stable")
     picks = sorted(set(int(order[min(n - 1, (k * (n - 1)) // 7)]) for k in range(8)))
+    dumped = dump_files(n) if a.dump_outputs and rank == 0 else []
+    wanted = set(picks) | set(dumped)
     got = {}
     if chunked:
+        # the ring keeps only the last two chunks of a pass: the outputs are taken from one more, identical pass
         def grab(chunk, f0, cnt, d_slot, ooff, osz, stat):
-            for i in picks:
+            for i in wanted:
                 if f0 <= i < f0 + cnt:
                     buf = C.create_string_buffer(int(osz[i - f0]))
                     ctx.d2h(buf, d_slot + int(ooff[i - f0]), len(buf))
                     got[i] = buf.raw
         batch.strip_chunked(stream=sptr, on_chunk=grab)
+        assert (batch.out_sizes[:n] == last_sizes).all() and (batch.status[:n] == last_status).all()
     else:
-        for i in picks:
+        for i in wanted:
             got[i] = batch.read_output(i)
+    if dumped:
+        write_dump(a.dump_outputs, last_sizes, last_status, dumped, got)
     pdir = tempfile.mkdtemp(prefix="lb2_par_%d_" % rank, dir=shm_dir())
     mismatches = 0
     for i in picks:
@@ -753,7 +797,12 @@ def main():
     ap.add_argument("--no-host-legs", action="store_true", help="skip cpu_baseline / tree / real_trees (N=1)")
     ap.add_argument("--no-real-trees", action="store_true")
     ap.add_argument("--profile-mode", action="store_true", help="device-resident steps only (for runs under ncu; not a bench value)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write rank 0's results of the last step to DIR/*.npy: out_sizes and status "
+                         "(float64, one per file) and a seeded sample of the stripped bytes (sample_files, sample_bytes as float32)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
