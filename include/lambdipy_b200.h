@@ -206,6 +206,54 @@ int lb2_corpus_fill(lb2_ctx *ctx, void *d_arena, const lb2_fill_region *h_region
 int lb2_corpus_scatter(lb2_ctx *ctx, void *d_arena, const void *h_data, uint64_t data_bytes, const uint64_t *h_dst,
                        const uint64_t *h_src, const uint64_t *h_len, uint32_t n);
 
+/* ---- gzip release tarballs (DEFLATE on the GPU) ------------------------------------------ */
+/* Replaces the compression of
+ *     with tarfile.open(tarball_path, "w:gz") as tar: tar.add(path, arcname=...)
+ *                                              /root/reference/lambdipy/package_build.py:165-172
+ * (zlib level 9, one CPU core).  The stream is cut into 64 KiB chunks compressed independently by one CTA
+ * each (back-references reach 32 KiB into the preceding input); every non-final chunk ends with an empty
+ * stored block.  The result inflates to exactly the input; its bytes differ from zlib's.  The output is a
+ * pure function of the input bytes (and, for lb2_gzip_segments, independent of the window size). */
+typedef struct lb2_gzip_stats {
+  uint64_t in_bytes, out_bytes;  /* uncompressed input, compressed output (deflate stream only)                 */
+  float kernel_ms;               /* deflate kernel + concatenation, CUDA events, summed over windows             */
+  double read_s;                 /* lb2_gzip_segments: pread + memcpy into the pinned slots, summed over workers  */
+  double upload_s;               /* wall time spent waiting for window uploads (window 0, then what compressing
+                                    the previous window did not hide)                                           */
+  double download_s, write_s;    /* D2H of the compressed output, pwrite of header / stream / trailer, wall       */
+  double setup_s;                /* buffer allocation inside this call (0 once the context's buffers are large enough) */
+  uint64_t n_chunks;
+  uint32_t n_windows, io_threads;
+  uint64_t phase_cycles[6];      /* SM cycles summed over CTAs: hash sort, scatter, match search, lazy parse,
+                                    Huffman + header, emit                                                      */
+} lb2_gzip_stats;
+
+/* Raw DEFLATE of n bytes at d_in (HBM) into d_out (cap bytes).  `hist` bytes before d_in (at most 32768
+ * are used) are history: back-references may reach into them, they are not emitted.  final != 0: the last
+ * block has BFINAL=1; final == 0: the stream ends with a sync flush and may be continued by a later call
+ * whose history is this call's last 32 KiB.  *crc32 = CRC-32 of the n bytes.  Synchronous on `stream`
+ * (NULL: the context's stream).  cap too small: LB2_E_CAPACITY, *out_len = bytes needed.  A bound for cap:
+ * ceil(n / 65536) * 66560 (or 66560 when n == 0). */
+int lb2_deflate_device(lb2_ctx *ctx, const void *d_in, uint64_t n, uint32_t hist, uint32_t final, void *d_out,
+                       uint64_t cap, uint64_t *out_len, uint32_t *crc32, lb2_gzip_stats *stats, void *stream);
+
+/* One piece of the uncompressed stream: `data` != NULL: len literal bytes; else the first len bytes of
+ * the regular file `path`. */
+typedef struct lb2_gz_segment {
+  const void *data;
+  const char *path;
+  uint64_t len;
+} lb2_gz_segment;
+/* Writes out_path = gz_header (gz_header_len bytes, as given), the DEFLATE stream of the concatenated
+ * segments, CRC-32 and ISIZE (little-endian, ISIZE mod 2^32).  The stream is processed in windows of
+ * LB2_GZ_WINDOW_MB (default 1024) MB, each primed with the previous window's last 32 KiB; reading window
+ * k+1 overlaps compressing and writing window k.  File bodies are read by lb2_strip_tree's I/O workers into its
+ * pinned slot ring (lb2_tree_prepare) and DMA'd into the window; the window buffers stay allocated with the
+ * context and are reused by later calls.  A file shorter than its segment (or unreadable) gives
+ * LB2_E_IO and out_path is removed. */
+int lb2_gzip_segments(lb2_ctx *ctx, const lb2_gz_segment *segs, uint32_t n_segs, const char *out_path,
+                      const void *gz_header, uint32_t gz_header_len, lb2_gzip_stats *stats);
+
 #ifdef __cplusplus
 }
 #endif

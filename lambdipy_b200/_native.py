@@ -24,6 +24,7 @@ EXPORTS = [
     "lb2_strip_device_async", "lb2_batch_results", "lb2_strip_host", "lb2_strip_tree",
     "lb2_plan_device", "lb2_corpus_fill", "lb2_corpus_scatter",
     "lb2_strip_device_chunked", "lb2_tree_prepare", "lb2_strip_tree_ex", "lb2_tree_cleanup",
+    "lb2_deflate_device", "lb2_gzip_segments",
 ]
 
 
@@ -54,6 +55,25 @@ class TreeStats(C.Structure):
         d = {k: getattr(self, k) for k, _ in self._fields_ if k != "batch"}
         d["batch"] = self.batch.as_dict()
         return d
+
+
+class GzipStats(C.Structure):
+    _fields_ = [
+        ("in_bytes", C.c_uint64), ("out_bytes", C.c_uint64), ("kernel_ms", C.c_float),
+        ("read_s", C.c_double), ("upload_s", C.c_double), ("download_s", C.c_double), ("write_s", C.c_double),
+        ("setup_s", C.c_double), ("n_chunks", C.c_uint64), ("n_windows", C.c_uint32), ("io_threads", C.c_uint32),
+        ("phase_cycles", C.c_uint64 * 6),
+    ]
+    PHASES = ("hash_sort", "scatter", "match", "parse", "huffman_header", "emit")
+
+    def as_dict(self):
+        d = {k: getattr(self, k) for k, _ in self._fields_ if k != "phase_cycles"}
+        d["phase_cycles"] = dict(zip(self.PHASES, list(self.phase_cycles)))
+        return d
+
+
+class GzSegment(C.Structure):
+    _fields_ = [("data", C.c_void_p), ("path", C.c_char_p), ("len", C.c_uint64)]
 
 
 class FillRegion(C.Structure):
@@ -130,6 +150,12 @@ def load():
     lib.lb2_tree_cleanup.restype = C.c_int
     lib.lb2_tree_prepare.argtypes = [vp, C.c_uint64]
     lib.lb2_tree_prepare.restype = C.c_int
+    lib.lb2_deflate_device.argtypes = [vp, vp, C.c_uint64, C.c_uint32, C.c_uint32, vp, C.c_uint64, u64p,
+                                       C.POINTER(C.c_uint32), C.POINTER(GzipStats), vp]
+    lib.lb2_deflate_device.restype = C.c_int
+    lib.lb2_gzip_segments.argtypes = [vp, C.POINTER(GzSegment), C.c_uint32, C.c_char_p, C.c_char_p, C.c_uint32,
+                                      C.POINTER(GzipStats)]
+    lib.lb2_gzip_segments.restype = C.c_int
     _lib = lib
     return lib
 

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "liblambdipy_b200.so")
-SOURCES = ["plan.cu", "compact.cu", "compact_tma.cu", "corpus.cu", "api.cu"]
+SOURCES = ["plan.cu", "compact.cu", "compact_tma.cu", "corpus.cu", "deflate.cu", "api.cu"]
 HEADERS = ["lb2_common.cuh", "copy_device.cuh", os.path.join("..", "..", "include", "lambdipy_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -80,6 +80,24 @@ struct lb2_ctx {
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_d2h[2] = {nullptr, nullptr}, ev_planned = nullptr;
   } slot[3];
   TreeEngine *tree = nullptr;  // lb2_strip_tree: pinned slot ring, I/O worker streams, HBM batch buffers
+  // lb2_deflate_device / lb2_gzip_segments: per-chunk output slots, per-CTA match scratch, concatenation tile list,
+  // and the window buffers of lb2_gzip_segments -- grown on demand and kept for the context's life, like the tree
+  // engine (whose pinned slot ring and worker streams upload the windows)
+  struct DeflateWs {
+    uint8_t *slots = nullptr;
+    uint32_t *size_crc = nullptr, *h_size_crc = nullptr;  // out_size[cap] | chunk_crc[cap], device and pinned
+    uint32_t *scratch = nullptr;
+    uint16_t *dists = nullptr;
+    Tile *tiles = nullptr;
+    BatchCounters *ctr = nullptr;
+    uint64_t *out_off = nullptr;
+    unsigned long long *phase = nullptr;  // DEFLATE_PHASES cycle counters
+    uint64_t cap_chunks = 0, cap_tiles = 0;
+    int grid = 0;
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    uint8_t *d_win[2] = {nullptr, nullptr}, *d_out = nullptr, *h_out = nullptr;  // window (+ 32 KiB history) x2, output
+    uint64_t cap_win[2] = {0, 0}, cap_out = 0, cap_h_out = 0;
+  } gz;
 };
 struct TreeEngine;
 static void tree_engine_free(TreeEngine *e);
@@ -383,6 +401,11 @@ void lb2_ctx_destroy(lb2_ctx *ctx) {
     if (sl.ev_planned) cudaEventDestroy(sl.ev_planned);
   }
   tree_engine_free(ctx->tree);
+  cudaFree(ctx->gz.slots); cudaFree(ctx->gz.size_crc); cudaFreeHost(ctx->gz.h_size_crc); cudaFree(ctx->gz.scratch);
+  cudaFree(ctx->gz.dists); cudaFree(ctx->gz.tiles); cudaFree(ctx->gz.ctr); cudaFree(ctx->gz.out_off);
+  cudaFree(ctx->gz.phase); cudaFree(ctx->gz.d_win[0]); cudaFree(ctx->gz.d_win[1]); cudaFree(ctx->gz.d_out);
+  cudaFreeHost(ctx->gz.h_out);
+  for (auto &e : ctx->gz.ev) if (e) cudaEventDestroy(e);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }
@@ -1448,6 +1471,344 @@ int lb2_corpus_scatter(lb2_ctx *ctx, void *d_arena, const void *h_data, uint64_t
   CK(cudaGetLastError());
   cudaFree(d_stage); cudaFree(d_tiles); cudaFree(d_ctr); cudaFree(d_off);
   return LB2_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------- gzip: chunk concatenation, CRC combine, windows
+
+// CRC-32 algebra (reflected polynomial 0xEDB88320): a * b mod P, and x^(8 n) mod P.  crc(A || B) =
+// (x^(8 |B|) * crc(A)) ^ crc(B) for the standard (pre- and post-inverted) CRC.
+static uint32_t crc_mulmod(uint32_t a, uint32_t b) {
+  uint32_t p = 0;
+  for (uint32_t m = 1u << 31; m; m >>= 1) {
+    if (a & m) p ^= b;
+    b = (b & 1) ? (b >> 1) ^ 0xEDB88320u : b >> 1;
+  }
+  return p;
+}
+static uint32_t crc_shift(uint64_t nbytes) {
+  uint32_t p = 1u << 31, sq = 1u << 23;
+  for (; nbytes; nbytes >>= 1) {
+    if (nbytes & 1) p = crc_mulmod(sq, p);
+    sq = crc_mulmod(sq, sq);
+  }
+  return p;
+}
+static uint32_t crc_combine(uint32_t c1, uint32_t c2, uint64_t len2) {
+  return len2 ? crc_mulmod(crc_shift(len2), c1) ^ c2 : c1;
+}
+
+
+static int deflate_reserve(lb2_ctx *ctx, uint64_t n_chunks) {
+  auto &g = ctx->gz;
+  if (!g.scratch) {
+    deflate_smem_setup();
+    CK(cudaGetLastError());
+    g.grid = ctx->sm_count;   // ~210 KB of shared memory per CTA: one CTA per SM
+    CK(cudaMalloc(&g.scratch, (size_t)g.grid * (DEFLATE_HIST + 2 * DEFLATE_CHUNK) * sizeof(uint32_t)));
+    CK(cudaMalloc(&g.dists, (size_t)g.grid * DEFLATE_CHUNK * sizeof(uint16_t)));
+    CK(cudaMalloc(&g.ctr, sizeof(BatchCounters)));
+    CK(cudaMalloc(&g.out_off, sizeof(uint64_t)));
+    CK(cudaMemset(g.out_off, 0, sizeof(uint64_t)));
+    CK(cudaMalloc(&g.phase, DEFLATE_PHASES * sizeof(unsigned long long)));
+    for (auto &e : g.ev) CK(cudaEventCreate(&e));
+  }
+  if (n_chunks > g.cap_chunks) {
+    cudaFree(g.slots); cudaFree(g.size_crc); cudaFreeHost(g.h_size_crc); cudaFree(g.tiles);
+    g.slots = nullptr; g.size_crc = nullptr; g.h_size_crc = nullptr; g.tiles = nullptr; g.cap_chunks = g.cap_tiles = 0;
+    // a slot's bytes land at any offset of the stream, so they can touch one 16 KiB tile boundary more than
+    // their length alone needs (a stored chunk, 65 551 bytes, can span 6 tiles)
+    const uint64_t tiles_per_chunk = (DEFLATE_SLOT + TILE_BYTES - 1) / TILE_BYTES + 1;
+    CK(cudaMalloc(&g.slots, n_chunks * DEFLATE_SLOT));
+    CK(cudaMalloc(&g.size_crc, n_chunks * 2 * sizeof(uint32_t)));
+    CK(cudaHostAlloc(&g.h_size_crc, n_chunks * 2 * sizeof(uint32_t), cudaHostAllocDefault));
+    CK(cudaMalloc(&g.tiles, n_chunks * tiles_per_chunk * sizeof(Tile)));
+    g.cap_chunks = n_chunks;
+    g.cap_tiles = n_chunks * tiles_per_chunk;
+  }
+  return LB2_OK;
+}
+
+static int deflate_run(lb2_ctx *ctx, const uint8_t *d_in, uint64_t n, uint32_t hist, bool final_, uint8_t *d_out,
+                       uint64_t cap, uint64_t *out_len, uint32_t *crc_out, lb2_gzip_stats *st, cudaStream_t s) {
+  uint64_t nch = (n + DEFLATE_CHUNK - 1) / DEFLATE_CHUNK;
+  if (!nch && final_) nch = 1;   // an empty final stream is one empty fixed block
+  *out_len = 0;
+  *crc_out = 0;
+  if (!nch) return LB2_OK;
+  int rc = deflate_reserve(ctx, nch);
+  if (rc) return rc;
+  auto &g = ctx->gz;
+  DeflateArgs a;
+  a.in = d_in; a.n = n; a.hist = std::min<uint32_t>(hist, DEFLATE_HIST); a.final_ = final_ ? 1 : 0;
+  a.n_chunks = (uint32_t)nch;
+  a.slots = g.slots; a.out_size = g.size_crc; a.chunk_crc = g.size_crc + nch;
+  a.scratch = g.scratch; a.dists = g.dists; a.phase_cycles = g.phase;
+  CK(cudaMemsetAsync(g.phase, 0, DEFLATE_PHASES * sizeof(unsigned long long), s));
+  CK(cudaEventRecord(g.ev[0], s));
+  launch_deflate(a, (int)std::min<uint64_t>(nch, (uint64_t)g.grid), s);
+  CK(cudaGetLastError());
+  CK(cudaEventRecord(g.ev[1], s));
+  CK(cudaMemcpyAsync(g.h_size_crc, g.size_crc, nch * 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+  unsigned long long phase[DEFLATE_PHASES];
+  CK(cudaMemcpyAsync(phase, g.phase, sizeof phase, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[1]));
+  // exclusive scan of the slot sizes -> one tile list for the compaction kernel (the copy path of the strip)
+  std::vector<Tile> tiles;
+  tiles.reserve(nch * 5);
+  uint64_t total = 0;
+  for (uint64_t c = 0; c < nch; c++) {
+    const uint64_t sz = g.h_size_crc[c];
+    const uint64_t src = reinterpret_cast<uint64_t>(g.slots) + c * DEFLATE_SLOT;
+    for (uint64_t k = 0; sz && k <= (total + sz - 1) / TILE_BYTES - total / TILE_BYTES; k++)
+      tiles.push_back(extent_tile(src, total, sz, 0, (uint32_t)k));
+    total += sz;
+  }
+  *out_len = total;
+  if (total > cap) { ctx->err = "deflate: output capacity " + std::to_string(cap) + " < " + std::to_string(total); return LB2_E_CAPACITY; }
+  if (!d_out && total) { ctx->err = "deflate: NULL output"; return LB2_E_ARG; }
+  if (tiles.size() > g.cap_tiles) {   // cannot happen with the bound above; never write past the list
+    ctx->err = "deflate: " + std::to_string(tiles.size()) + " concatenation tiles > " + std::to_string(g.cap_tiles);
+    return LB2_E_STATE;
+  }
+  if (!tiles.empty()) {
+    BatchCounters bc;
+    memset(&bc, 0, sizeof bc);
+    bc.n_tiles = tiles.size();
+    CK(cudaMemcpyAsync(g.tiles, tiles.data(), tiles.size() * sizeof(Tile), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(g.ctr, &bc, sizeof bc, cudaMemcpyHostToDevice, s));
+    CompactArgs ca;
+    ca.tiles = g.tiles; ca.ctr = g.ctr; ca.out_off = g.out_off; ca.out = d_out;
+    ca.rebase_lo = ca.rebase_len = ca.rebase_delta = 0;
+    CK(cudaEventRecord(g.ev[0], s));
+    launch_compact(ca, ctx->sm_count * 4, s);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(g.ev[1], s));
+    CK(cudaStreamSynchronize(s));
+    float ms2 = 0;
+    CK(cudaEventElapsedTime(&ms2, g.ev[0], g.ev[1]));
+    ms += ms2;
+  }
+  // chunks are DEFLATE_CHUNK bytes except the last: one fixed shift operator folds them
+  const uint32_t op = crc_shift(DEFLATE_CHUNK);
+  const uint32_t *cc = g.h_size_crc + nch;
+  uint32_t crc = cc[0];
+  for (uint64_t c = 1; c < nch; c++) {
+    const uint64_t len = std::min<uint64_t>(DEFLATE_CHUNK, n - c * DEFLATE_CHUNK);
+    crc = (len == DEFLATE_CHUNK ? crc_mulmod(op, crc) : crc_mulmod(crc_shift(len), crc)) ^ cc[c];
+  }
+  *crc_out = n ? crc : 0;
+  if (st) {
+    st->in_bytes += n; st->out_bytes += total; st->kernel_ms += ms; st->n_chunks += nch;
+    for (int k = 0; k < DEFLATE_PHASES; k++) st->phase_cycles[k] += phase[k];
+  }
+  return LB2_OK;
+}
+
+// The concatenated segments of one lb2_gzip_segments call.  fill() is called from several I/O workers at once.
+struct GzSource {
+  const lb2_gz_segment *segs;
+  uint32_t n_segs;
+  std::vector<uint64_t> off;  // n_segs + 1 prefix sums
+  // bytes [start, start + len) -> dst; "" or an error message
+  std::string fill(uint8_t *dst, uint64_t start, uint64_t len) const {
+    uint32_t i = (uint32_t)(std::upper_bound(off.begin(), off.end(), start) - off.begin()) - 1;
+    uint64_t done = 0;
+    for (; done < len && i < n_segs; i++) {
+      const uint64_t in_seg = start + done - off[i];
+      const uint64_t take = std::min(segs[i].len - in_seg, len - done);
+      if (!take) continue;
+      if (segs[i].data) {
+        memcpy(dst + done, static_cast<const uint8_t *>(segs[i].data) + in_seg, take);
+      } else {
+        const int f = open(segs[i].path, O_RDONLY | O_CLOEXEC);
+        if (f < 0) return std::string("open ") + segs[i].path + ": " + strerror(errno);
+        const bool ok = pread_all(f, dst + done, take, in_seg);
+        close(f);
+        if (!ok) return std::string("short read (file changed since it was recorded?): ") + segs[i].path;
+      }
+      done += take;
+    }
+    return done == len ? "" : "segments shorter than their recorded total";
+  }
+};
+
+// Bytes [start, start + len) of the source -> d_dst, through the tree engine's pinned slot ring: piece j
+// (slot_bytes each) is read by I/O worker j % n_workers into one of its two slots and DMA'd on its stream.
+// Returns LB2_OK, LB2_E_IO or LB2_E_CUDA (message in *err); *read_s += pread/memcpy time summed over workers.
+static int gz_upload(lb2_ctx *ctx, const GzSource &src, uint64_t start, uint64_t len, uint8_t *d_dst, std::string *err,
+                     double *read_s) {
+  TreeEngine &E = *ctx->tree;
+  const uint64_t sb = E.slot_bytes, n_pieces = (len + sb - 1) / sb;
+  const int nw = (int)std::min<uint64_t>((uint64_t)E.n_workers, std::max<uint64_t>(1, n_pieces));
+  std::vector<int> rc(nw, LB2_OK);
+  std::vector<std::string> msg(nw);
+  std::vector<double> rs(nw, 0.0);
+  std::vector<std::thread> pool;
+  for (int wi = 0; wi < nw; wi++)
+    pool.emplace_back([&, wi] {
+      cudaSetDevice(ctx->device);
+      TreeWorker &w = E.workers[wi];
+      for (uint64_t j = wi; j < n_pieces && rc[wi] == LB2_OK; j += nw) {
+        uint8_t *slot = E.h_ring + ((uint64_t)wi * 2 + (w.k & 1)) * sb;
+        cudaEvent_t ev = w.ev[w.k & 1];
+        w.k++;
+        if (cudaEventSynchronize(ev) != cudaSuccess) { rc[wi] = LB2_E_CUDA; msg[wi] = "gzip: slot DMA failed"; break; }
+        const uint64_t o = j * sb, l = std::min(sb, len - o);
+        const double t0 = now_s();
+        msg[wi] = src.fill(slot, start + o, l);
+        rs[wi] += now_s() - t0;
+        if (!msg[wi].empty()) { rc[wi] = LB2_E_IO; break; }
+        if (cudaMemcpyAsync(d_dst + o, slot, l, cudaMemcpyHostToDevice, w.stream) != cudaSuccess ||
+            cudaEventRecord(ev, w.stream) != cudaSuccess) { rc[wi] = LB2_E_CUDA; msg[wi] = "gzip: slot DMA failed"; }
+      }
+      if (cudaStreamSynchronize(w.stream) != cudaSuccess && rc[wi] == LB2_OK) { rc[wi] = LB2_E_CUDA; msg[wi] = "gzip: slot DMA failed"; }
+    });
+  for (auto &t : pool) t.join();
+  for (double r : rs) *read_s += r;
+  for (int wi = 0; wi < nw; wi++)
+    if (rc[wi] != LB2_OK) { *err = msg[wi]; return rc[wi]; }
+  return LB2_OK;
+}
+
+static int grow_dev(lb2_ctx *ctx, uint8_t **p, uint64_t *cap, uint64_t need) {
+  if (*cap >= need) return LB2_OK;
+  cudaFree(*p); *p = nullptr; *cap = 0;
+  CK(cudaMalloc(p, need));
+  *cap = need;
+  return LB2_OK;
+}
+
+extern "C" {
+
+int lb2_deflate_device(lb2_ctx *ctx, const void *d_in, uint64_t n, uint32_t hist, uint32_t final_, void *d_out,
+                       uint64_t cap, uint64_t *out_len, uint32_t *crc32, lb2_gzip_stats *stats, void *stream) {
+  if (!ctx || (!d_in && (n || hist)) || !out_len || !crc32) { if (ctx) ctx->err = "NULL argument"; return LB2_E_ARG; }
+  CK(cudaSetDevice(ctx->device));
+  if (stats) memset(stats, 0, sizeof *stats);
+  cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+  int rc = deflate_run(ctx, static_cast<const uint8_t *>(d_in), n, hist, final_ != 0, static_cast<uint8_t *>(d_out), cap,
+                       out_len, crc32, stats, s);
+  if (stats) stats->n_windows = 1;
+  return rc;
+}
+
+int lb2_gzip_segments(lb2_ctx *ctx, const lb2_gz_segment *segs, uint32_t n_segs, const char *out_path,
+                      const void *gz_header, uint32_t gz_header_len, lb2_gzip_stats *stats) {
+  if (!ctx || !out_path || (n_segs && !segs) || (gz_header_len && !gz_header)) { if (ctx) ctx->err = "NULL argument"; return LB2_E_ARG; }
+  for (uint32_t i = 0; i < n_segs; i++)
+    if (!segs[i].data && !segs[i].path && segs[i].len) { ctx->err = "segment without data or path"; return LB2_E_ARG; }
+  CK(cudaSetDevice(ctx->device));
+  lb2_gzip_stats st;
+  memset(&st, 0, sizeof st);
+  GzSource src{segs, n_segs, std::vector<uint64_t>(n_segs + 1, 0)};
+  for (uint32_t i = 0; i < n_segs; i++) src.off[i + 1] = src.off[i] + segs[i].len;
+  const uint64_t total = src.off[n_segs];
+  uint64_t W = env_u64("LB2_GZ_WINDOW_MB", 1024) << 20;
+  W = std::max<uint64_t>(DEFLATE_CHUNK, W / DEFLATE_CHUNK * DEFLATE_CHUNK);
+  W = std::min<uint64_t>(W, std::max<uint64_t>(DEFLATE_CHUNK, (total + DEFLATE_CHUNK - 1) / DEFLATE_CHUNK * DEFLATE_CHUNK));
+  const uint64_t n_win = std::max<uint64_t>(1, (total + W - 1) / W);
+  const uint64_t out_cap = W / DEFLATE_CHUNK * DEFLATE_SLOT;
+  constexpr uint64_t H_OUT = 64ull << 20;   // pinned bounce buffer of the compressed output
+  cudaStream_t s = ctx->stream;
+  auto &g = ctx->gz;
+
+  int rc = LB2_OK;
+  double t0 = now_s();
+  if (!ctx->tree) rc = tree_engine_prepare(ctx, 0);
+  for (int b = 0; rc == LB2_OK && b < (n_win > 1 ? 2 : 1); b++) rc = grow_dev(ctx, &g.d_win[b], &g.cap_win[b], DEFLATE_HIST + W);
+  if (rc == LB2_OK) rc = grow_dev(ctx, &g.d_out, &g.cap_out, out_cap);
+  if (rc == LB2_OK && !g.h_out) {
+    cudaError_t e = cudaHostAlloc(&g.h_out, H_OUT, cudaHostAllocDefault);
+    if (e != cudaSuccess) { ctx->err = std::string("cudaHostAlloc(gzip output): ") + cudaGetErrorString(e); rc = LB2_E_CUDA; }
+    else g.cap_h_out = H_OUT;
+  }
+  st.setup_s = now_s() - t0;
+  st.io_threads = ctx->tree ? (uint32_t)ctx->tree->n_workers : 0;
+  if (rc != LB2_OK) { if (stats) *stats = st; return rc; }
+
+  int fd = open(out_path, O_WRONLY | O_CREAT | O_TRUNC | O_CLOEXEC, 0644);
+  if (fd < 0) { ctx->err = std::string("open ") + out_path + ": " + strerror(errno); if (stats) *stats = st; return LB2_E_IO; }
+  auto fail = [&](int code, const std::string &m) { if (rc == LB2_OK) { if (!m.empty()) ctx->err = m; rc = code; } };
+  std::thread uploader;
+  int up_rc = LB2_OK;
+  std::string up_err;
+  double read_s = 0;
+  do {
+    uint64_t pos = 0;
+    t0 = now_s();
+    if (!pwrite_all(fd, static_cast<const uint8_t *>(gz_header), gz_header_len, 0)) { fail(LB2_E_IO, "write header"); break; }
+    pos = gz_header_len;
+    st.write_s += now_s() - t0;
+    t0 = now_s();
+    up_rc = gz_upload(ctx, src, 0, std::min(W, total), g.d_win[0] + DEFLATE_HIST, &up_err, &read_s);
+    st.upload_s += now_s() - t0;
+    if (up_rc != LB2_OK) { fail(up_rc, up_err); break; }
+    uint32_t crc = 0;
+    uint64_t prev_len = 0;
+    for (uint64_t k = 0; k < n_win && rc == LB2_OK; k++) {
+      const int b = (int)(k & 1);
+      const uint64_t wlen = std::min(W, total - k * W);
+      uint8_t *d_in = g.d_win[b] + DEFLATE_HIST;
+      // the last 32 KiB of window k-1 become the history in front of window k
+      const uint32_t hist = (uint32_t)std::min<uint64_t>(DEFLATE_HIST, k * W);
+      cudaError_t e = cudaSuccess;
+      if (hist && ((e = cudaMemcpyAsync(d_in - hist, g.d_win[1 - b] + DEFLATE_HIST + prev_len - hist, hist,
+                                        cudaMemcpyDeviceToDevice, s)) != cudaSuccess ||
+                   (e = cudaStreamSynchronize(s)) != cudaSuccess)) {
+        fail(LB2_E_CUDA, std::string("gzip history copy: ") + cudaGetErrorString(e));
+        break;
+      }
+      // window k+1 is read and uploaded (into the other buffer, behind the history copy above) while k is compressed
+      if (k + 1 < n_win)
+        uploader = std::thread([&, k, b] {
+          cudaSetDevice(ctx->device);
+          up_rc = gz_upload(ctx, src, (k + 1) * W, std::min(W, total - (k + 1) * W), g.d_win[1 - b] + DEFLATE_HIST, &up_err, &read_s);
+        });
+      uint64_t olen = 0;
+      uint32_t wcrc = 0;
+      int r = deflate_run(ctx, d_in, wlen, hist, k + 1 == n_win, g.d_out, out_cap, &olen, &wcrc, &st, s);
+      if (r) fail(r, "");
+      for (uint64_t o = 0; rc == LB2_OK && o < olen; o += g.cap_h_out) {
+        const uint64_t l = std::min(g.cap_h_out, olen - o);
+        t0 = now_s();
+        if ((e = cudaMemcpyAsync(g.h_out, g.d_out + o, l, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
+            (e = cudaStreamSynchronize(s)) != cudaSuccess) {
+          fail(LB2_E_CUDA, std::string("gzip download: ") + cudaGetErrorString(e));
+          break;
+        }
+        st.download_s += now_s() - t0;
+        t0 = now_s();
+        if (!pwrite_all(fd, g.h_out, l, pos + o)) fail(LB2_E_IO, std::string("write ") + out_path + ": " + strerror(errno));
+        st.write_s += now_s() - t0;
+      }
+      pos += olen;
+      crc = crc_combine(crc, wcrc, wlen);
+      t0 = now_s();
+      if (uploader.joinable()) uploader.join();
+      st.upload_s += now_s() - t0;   // the part of the next window's upload the compression did not hide
+      if (up_rc != LB2_OK) fail(up_rc, up_err);
+      prev_len = wlen;
+      st.n_windows++;
+    }
+    if (rc != LB2_OK) break;
+    uint8_t trailer[8];
+    const uint32_t isize = (uint32_t)total;
+    for (int i = 0; i < 4; i++) { trailer[i] = (uint8_t)(crc >> (8 * i)); trailer[4 + i] = (uint8_t)(isize >> (8 * i)); }
+    t0 = now_s();
+    if (!pwrite_all(fd, trailer, 8, pos) || ftruncate(fd, (off_t)(pos + 8)) != 0) { fail(LB2_E_IO, "write trailer"); break; }
+    st.write_s += now_s() - t0;
+  } while (0);
+
+  if (uploader.joinable()) uploader.join();
+  if (close(fd) != 0) fail(LB2_E_IO, std::string("close ") + out_path + ": " + strerror(errno));
+  if (rc != LB2_OK) unlink(out_path);
+  st.read_s = read_s;
+  if (stats) *stats = st;
+  return rc;
 }
 
 }  // extern "C"
